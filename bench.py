@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N --steps K --warmup W]         the CUDA path (one process per GPU under torchrun)
   python bench.py --impl reference [...]                  the CPU implementation timed on the host cores
+  python bench.py [...] --dump-outputs DIR                also write what the last timed step computed as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one synthetic batch: BASELINE.json configs[2]
 (65 536 prompts, lengths uniform 8..4096 B, cl100k pattern) -- the config the north_star metric
@@ -218,6 +219,30 @@ def tiktoken_context_rate(data, offs, rv, threads, target_s=6.0):
             "sample": "first %d prompts (%d bytes), %.1f s wall" % (k, b, t)}
 
 
+DUMP_SEED = 20261017
+DUMP_ID_BYTES = 15 << 20      # input bytes whose ids are written: a token covers at least one byte, so at most 60 MiB of ids
+
+
+def dump_outputs(out_dir, offs, d_ids, d_out_off, d_counts):
+    """Write what the device leg hands its caller, so that two builds can be compared output for output: the token offsets of
+    every prompt (float64: they pass 2**24), the per-prompt token counts, and the ids of a fixed sample of prompts holding
+    DUMP_ID_BYTES of input (ids stay below 2**24, exact in float32), with the sample's prompt indices.  The sample is drawn
+    from the inputs alone, so equal inputs give equal samples whatever the build computes."""
+    import torch
+    n = len(offs) - 1
+    out_off = d_out_off.cpu().numpy()
+    order = np.random.default_rng(DUMP_SEED).permutation(n)
+    in_bytes = np.cumsum(np.diff(offs.astype(np.int64))[order])
+    pick = np.sort(order[:max(1, int(np.searchsorted(in_bytes, DUMP_ID_BYTES, side="right")))])
+    pos = np.concatenate([np.arange(out_off[i], out_off[i + 1]) for i in pick])
+    ids = d_ids[torch.from_numpy(pos).to(d_ids.device)].cpu().numpy().view(np.uint32)
+    arrays = {"token_offsets": out_off.astype(np.float64), "token_counts": d_counts.cpu().numpy().astype(np.float32),
+              "sample_prompts": pick.astype(np.float64), "sample_ids": ids.astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """--impl reference: the CPU implementation on the host cores.  The reference tree has no tokenizer to
     compile (SURVEY.md F1), so this is the oracle port (oracle/bpe_oracle.c) on every host thread."""
@@ -269,6 +294,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-config5", action="store_true", help="skip the extra config-5 record")
     ap.add_argument("--sustain-seconds", type=float, default=2.0, help="extra record: the device leg held this long (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps of the device leg, write what its last step "
+                    "computed (rank 0's shard) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "cfbpe" else args.warmup
     if args.impl == "reference":
@@ -377,6 +404,8 @@ def main():
     total_all = sum_over_ranks(float(total))
     tokens_all = sum_over_ranks(float(n_tokens))
     value = total_all * args.steps / (dev_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, offs, d_ids, d_out_off, d_counts)
 
     # ---- the same leg held for ~2 s (the K timed steps above are tens of milliseconds): a sustained rate under sustained clocks
     sustained = None
