@@ -15,14 +15,16 @@ PATTERN_CL100K, PATTERN_O200K, PATTERN_LLAMA3, PATTERN_TEKKEN = 0, 1, 2, 3
 PATTERN_IDS = {"cl100k": 0, "o200k": 1, "llama3": 2, "tekken": 3}
 MAX_VOCABS = 8
 NUM_KERNELS = 10
-KERNEL_NAMES = ["pretok_split", "bpe_encode", "bpe_long", "flag_count", "tile_scan", "emit_compact", "bpe_list", "long_scan", "bpe_merge", "reserved"]
+KERNEL_NAMES = ["pretok_split", "bpe_encode", "bpe_long", "flag_count", "tile_scan", "emit_compact", "bpe_list", "long_scan", "bpe_merge", "window"]
+KEEP_HEAD, KEEP_TAIL = 0, 1
+KEEP = {"head": KEEP_HEAD, "tail": KEEP_TAIL}
 
 # every symbol include/cfbpe.h declares (checked by tests/test_abi.py without a GPU)
 EXPORTS = [
     "cfbpe_abi_version", "cfbpe_build_id", "cfbpe_create", "cfbpe_destroy", "cfbpe_last_error", "cfbpe_vocab_load",
     "cfbpe_vocab_get_info", "cfbpe_vocab_export", "cfbpe_vocab_import", "cfbpe_encode_batch", "cfbpe_count_batch",
     "cfbpe_encode_batch_device", "cfbpe_device_status", "cfbpe_host_alloc", "cfbpe_host_free",
-    "cfbpe_profile_enable", "cfbpe_profile_read", "cfbpe_decode_batch",
+    "cfbpe_profile_enable", "cfbpe_profile_read", "cfbpe_decode_batch", "cfbpe_encode_truncated", "cfbpe_encode_truncated_device",
 ]
 
 
@@ -97,6 +99,11 @@ def load():
     L.cfbpe_encode_batch_device.restype = C.c_int
     L.cfbpe_encode_batch_device.argtypes = [vp, C.c_uint32, vp, C.c_uint64, vp, vp, vp, C.c_uint64, vp, vp,
                                             C.POINTER(C.c_uint64), vp]
+    L.cfbpe_encode_truncated.restype = C.c_int
+    L.cfbpe_encode_truncated.argtypes = [vp, C.c_uint32, u8p, vp, u8p, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, vp, vp, vp]
+    L.cfbpe_encode_truncated_device.restype = C.c_int
+    L.cfbpe_encode_truncated_device.argtypes = [vp, C.c_uint32, vp, C.c_uint64, vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, vp, vp,
+                                                vp, vp, vp]
     L.cfbpe_device_status.restype = C.c_int
     L.cfbpe_device_status.argtypes = [vp, vp]
     L.cfbpe_host_alloc.restype = vp
@@ -245,6 +252,28 @@ class Context:
                                              vid, out_counts.ctypes.data))
         return out_counts[:n]
 
+    def encode_truncated(self, data: np.ndarray, offsets: np.ndarray, vocab_ids=None, *, max_tokens, keep=KEEP_HEAD, pad_id=0,
+                         budgets=None, want_ids=True):
+        """Every prompt cut to k_i = min(count_i, budgets[i], max_tokens) tokens (include/cfbpe.h: cfbpe_encode_truncated).
+        keep: KEEP_HEAD | KEEP_TAIL (or "head" | "tail").  Returns (rows uint32 [n, max_tokens] | None without want_ids, kept uint32 n,
+        counts uint32 n (untruncated), cut uint64 n (byte offset of the cut inside each prompt))."""
+        n = self._check_inputs(data, offsets, vocab_ids)
+        keep = KEEP.get(keep, keep) if isinstance(keep, str) else int(keep)
+        if budgets is not None:
+            if not isinstance(budgets, np.ndarray) or budgets.dtype != np.uint32 or budgets.ndim != 1 or len(budgets) != n or not budgets.flags.c_contiguous:
+                raise NativeError(EINVAL, "budgets must be a C-contiguous uint32 array with one entry per prompt")
+        rows = np.empty((n, int(max_tokens)), dtype=np.uint32) if want_ids and max_tokens > 0 else None
+        kept = np.empty(max(n, 1), dtype=np.uint32)
+        counts = np.empty(max(n, 1), dtype=np.uint32)
+        cut = np.empty(max(n, 1), dtype=np.uint64)
+        vid = None if vocab_ids is None else vocab_ids.ctypes.data
+        rc = load().cfbpe_encode_truncated(self._h, n, data.ctypes.data if data.size else None, offsets.ctypes.data, vid, int(max_tokens),
+                                           keep, int(pad_id), None if budgets is None else budgets.ctypes.data,
+                                           None if rows is None or not rows.size else rows.ctypes.data, kept.ctypes.data,
+                                           counts.ctypes.data, cut.ctypes.data)
+        self._check(rc)
+        return rows, kept[:n], counts[:n], cut[:n]
+
     def decode_batch(self, ids: np.ndarray, id_offsets: np.ndarray, vocab_ids=None, out_cap=None, out_bytes=None, out_offsets=None):
         """ids (uint32, packed) + id_offsets (uint64, n+1) -> (bytes uint8, byte offsets uint64 n+1).
         out_bytes / out_offsets: caller's buffers (pinned ones make the download several times faster)"""
@@ -276,6 +305,13 @@ class Context:
                                               C.byref(nt) if sync else None, stream)
         self._check(rc)
         return nt.value if sync else None
+
+    def encode_truncated_device(self, n_prompts, d_bytes, total_bytes, d_offsets, d_vocab_ids, max_tokens, keep, pad_id, d_budgets,
+                                d_out_rows, d_out_kept, d_out_counts, d_out_cut, stream=0):
+        """asynchronous, as encode_batch_device(sync=False): errors come from device_status"""
+        self._check(load().cfbpe_encode_truncated_device(self._h, n_prompts, d_bytes, total_bytes, d_offsets, d_vocab_ids, int(max_tokens),
+                                                         int(keep), int(pad_id), d_budgets, d_out_rows, d_out_kept, d_out_counts,
+                                                         d_out_cut, stream))
 
     def device_status(self, stream=0):
         self._check(load().cfbpe_device_status(self._h, stream))

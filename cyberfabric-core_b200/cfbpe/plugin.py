@@ -117,6 +117,29 @@ class CountTokensRequest:
 
 
 @dataclass
+class TruncateBatchRequest:
+    """every prompt cut to k_i = min(count_i, budgets[i], max_tokens) tokens: its first k_i (keep="head") or its last (keep="tail")"""
+    vocab: VocabRef
+    bytes: np.ndarray
+    offsets: np.ndarray
+    max_tokens: int                          # L >= 1: ids per row
+    keep: str = "head"                       # "head" | "tail"
+    pad_id: int = 0
+    budgets: Optional[np.ndarray] = None     # uint32, n, or None (max_tokens for every prompt)
+    want_ids: bool = True                    # False: kept counts and cuts only, no id leaves the device
+    vocabs_per_prompt: Optional[Sequence[VocabRef]] = None
+    vocab_index: Optional[np.ndarray] = None
+
+
+@dataclass
+class TruncateBatchResponse:
+    rows: Optional[np.ndarray]   # uint32 [n, max_tokens]: row i = its kept ids left-aligned, then pad_id; None without want_ids
+    kept: np.ndarray             # uint32, n: k_i
+    counts: np.ndarray           # uint32, n: the untruncated counts
+    cut: np.ndarray              # uint64, n: byte offset of the cut inside prompt i (head: the kept text is prompt[:cut], tail: prompt[cut:])
+
+
+@dataclass
 class DecodeBatchRequest:
     vocab: VocabRef
     ids: np.ndarray              # uint32, packed ids of all sequences
@@ -187,6 +210,9 @@ class TokenizerPluginClient:
         raise NotImplementedError
 
     def decode_batch(self, ctx: SecurityContext, req: "DecodeBatchRequest") -> "DecodeBatchResponse":
+        raise NotImplementedError
+
+    def truncate_batch(self, ctx: SecurityContext, req: "TruncateBatchRequest") -> "TruncateBatchResponse":
         raise NotImplementedError
 
 
@@ -360,6 +386,18 @@ class GpuBpeTokenizerPlugin(TokenizerPluginClient):
         except N.NativeError as e:
             raise _map_native(e) from e
 
+    def truncate_batch(self, ctx: SecurityContext, req: TruncateBatchRequest) -> TruncateBatchResponse:
+        self._check_arrays(req)
+        if req.keep not in N.KEEP:
+            raise InvalidInput("keep must be 'head' or 'tail', not %r" % (req.keep,))
+        vid = self._vocab_ids(req)
+        try:
+            rows, kept, counts, cut = self.ctx.encode_truncated(req.bytes, req.offsets, vid, max_tokens=req.max_tokens, keep=N.KEEP[req.keep],
+                                                                pad_id=req.pad_id, budgets=req.budgets, want_ids=req.want_ids)
+        except N.NativeError as e:
+            raise _map_native(e) from e
+        return TruncateBatchResponse(rows, kept, counts, cut)
+
     def decode_batch(self, ctx: SecurityContext, req: DecodeBatchRequest) -> DecodeBatchResponse:
         if req.ids.dtype != np.uint32 or req.offsets.dtype != np.uint64 or len(req.offsets) < 1:
             raise InvalidInput("ids must be uint32 and offsets uint64 with n+1 entries")
@@ -509,6 +547,17 @@ class LlmGatewayTokenizerService:
             parts = [enc[i] if kind == "s" else np.array([i], dtype=np.uint32) for kind, i in steps]
             out.append(np.concatenate(parts).astype(np.uint32) if parts else np.zeros(0, dtype=np.uint32))
         return out
+
+    def truncate(self, ctx: SecurityContext, model: str, texts: Sequence[str], max_tokens: int, keep: str = "head") -> List[Tuple[np.ndarray, int]]:
+        """Each text cut to at most max_tokens tokens: its first ones (keep="head") or its last ones (keep="tail").  Returns per text
+        (kept ids, byte cut): head keeps text.encode()[:cut], tail keeps text.encode()[cut:].
+        Two caveats.  The kept ids are a slice of the text's full encoding, and re-encoding the kept bytes need not give the same
+        ids: the pre-tokenizer's lookahead (\\s+(?!\\S)) sees different text at the cut.  And the cut is the token boundary as it is:
+        byte-level tokens split CJK characters and emoji, so it can fall inside a multi-byte UTF-8 character (the kept bytes then
+        do not decode as UTF-8 on their own)."""
+        data, offs = pack_texts(texts)
+        r = self._plugin().truncate_batch(ctx, TruncateBatchRequest(VocabRef(model), data, offs, max_tokens, keep))
+        return [(r.rows[i, :int(r.kept[i])].copy(), int(r.cut[i])) for i in range(len(texts))]
 
     def check_budget(self, ctx: SecurityContext, model: str, messages: Sequence[dict], remaining_tokens: int) -> bool:
         """pre-call estimate used by check_budget (modules/llm-gateway/docs/DESIGN.md:833-855)"""

@@ -1558,6 +1558,26 @@ tile_scan_kernel(const uint32_t* __restrict__ tile_counts, uint32_t n_tiles, uin
     if (threadIdx.x == 0 && status) { status->n_tokens = total; status->tok_end = base0 + total; }
 }
 
+// The id of the token whose first byte is bit `bit` of flag word w (emit_compact_kernel, emit_window_kernel).  bits / pb: the
+// token and piece flags of the word, prev_*: those of the word before; prank: the rank of the first piece that starts in word w.
+__device__ __forceinline__ uint32_t token_id_at(const DenseIds& dn, const uint32_t* __restrict__ ids_by_pos, uint64_t w, uint32_t bit,
+                                                uint32_t bits, uint32_t pb, uint32_t prev_bits, uint32_t prev_pb, uint64_t prank) {
+    const uint32_t below = pb & ((2u << bit) - 1u);                     // piece starts at or before this token, in my word
+    const uint32_t nb = __popc(below);
+    const uint32_t v = dn.by_piece[prank + nb - 1];                     // the piece this token belongs to
+    uint32_t id;
+    if (v == kPieceLong) id = ids_by_pos[(w << 5) + bit];               // a long piece: its kernel left the ids by position
+    else if (!(v & kPieceMulti)) id = v;                                // the piece is one token
+    else {                                                              // k-th token of a merged piece
+        uint32_t k;
+        const uint32_t before = bits & ((1u << bit) - 1u);              // tokens before me in my word
+        if (nb) { const uint32_t q = 31u - static_cast<uint32_t>(__clz(below)); k = __popc(before >> q); }
+        else { const uint32_t q = 31u - static_cast<uint32_t>(__clz(prev_pb)); k = __popc(prev_bits >> q) + __popc(before); }   // (a short piece starts at most one word back)
+        id = dn.extras[(v & ~kPieceMulti) + k];
+    }
+    return id;
+}
+
 __global__ void __launch_bounds__(256)
 emit_compact_kernel(const uint32_t* __restrict__ tok_bits, const uint32_t* __restrict__ piece_bits, uint64_t n_words,
                     const uint64_t* __restrict__ tile_base, DenseIds dn, const uint32_t* __restrict__ ids_by_pos,
@@ -1591,19 +1611,7 @@ emit_compact_kernel(const uint32_t* __restrict__ tok_bits, const uint32_t* __res
     while (rest) {
         const uint32_t bit = __ffs(rest) - 1;
         rest &= rest - 1;
-        const uint32_t below = pb & ((2u << bit) - 1u);                     // piece starts at or before this token, in my word
-        const uint32_t nb = __popc(below);
-        const uint32_t v = dn.by_piece[prank + nb - 1];                     // the piece this token belongs to
-        uint32_t id;
-        if (v == kPieceLong) id = ids_by_pos[(w << 5) + bit];               // a long piece: its kernel left the ids by position
-        else if (!(v & kPieceMulti)) id = v;                                // the piece is one token
-        else {                                                              // k-th token of a merged piece
-            uint32_t k;
-            const uint32_t before = bits & ((1u << bit) - 1u);              // tokens before me in my word
-            if (nb) { const uint32_t q = 31u - static_cast<uint32_t>(__clz(below)); k = __popc(before >> q); }
-            else { const uint32_t q = 31u - static_cast<uint32_t>(__clz(prev_pb)); k = __popc(prev_bits >> q) + __popc(before); }   // (a short piece starts at most one word back)
-            id = dn.extras[(v & ~kPieceMulti) + k];
-        }
+        const uint32_t id = token_id_at(dn, ids_by_pos, w, bit, bits, pb, prev_bits, prev_pb, prank);
         if (r < out_cap) out_ids[r] = id;
         ++r;
     }

@@ -36,6 +36,7 @@ struct ProfEvents {
     cudaEvent_t ev[CFBPE_NUM_KERNELS][2];
     cudaEvent_t h2d[2], d2h[2], total[2];
     bool launched[CFBPE_NUM_KERNELS];
+    uint32_t window_launches;            // K_WINDOW: window_select, + emit_window when rows are wanted
 };
 static inline void prof_mark(ProfEvents* p, int idx, cudaStream_t s, bool begin) {
     if (!p) return;
@@ -113,6 +114,9 @@ struct Lane {
     uint32_t* d_out_ids = nullptr;
     uint64_t* d_out_offsets = nullptr;
     uint32_t* d_out_counts = nullptr;
+    uint32_t* d_budgets = nullptr;        // truncated host calls: per-prompt budgets ...
+    uint32_t* d_kept = nullptr;           // ... kept counts ...
+    uint64_t* d_cut = nullptr;            // ... and cuts (the rows are staged in d_out_ids)
     Workspace ws{};
     DeviceStatus* h_status = nullptr;  // pinned
     ProfEvents prof{};
@@ -173,6 +177,32 @@ thread_local std::string tl_err;
 thread_local cfbpe_profile tl_profile{};
 thread_local bool tl_profile_ready = false;
 thread_local Lane* tl_device_lane = nullptr;      // the lane of this thread's last device-path call (cfbpe_device_status)
+
+// a truncated host call (cfbpe_encode_truncated): the window's parameters and the caller's buffers for its results (counts go
+// through the out_counts of the shared path)
+struct HostWindow {
+    uint32_t max_tokens, keep, pad_id;
+    const uint32_t* budgets;   // [n] or nullptr
+    uint32_t* rows;            // [n * max_tokens] or nullptr
+    uint32_t* kept;            // [n]
+    uint64_t* cut;             // [n] or nullptr
+};
+
+// the window of the prompts [p0, p0 + n) of a lane's buffers: the rows are staged in d_out_ids at p * L
+WindowView lane_window(Lane* ln, const HostWindow& hw, uint32_t p0) {
+    return WindowView{hw.max_tokens, hw.keep, hw.pad_id, hw.budgets ? ln->d_budgets + p0 : nullptr,
+                      hw.rows ? ln->d_out_ids + static_cast<uint64_t>(p0) * hw.max_tokens : nullptr, ln->d_kept + p0, nullptr,
+                      hw.cut ? ln->d_cut + p0 : nullptr};
+}
+// download the window results of prompts [p0, p0 + n) of a lane (its prompt p0 is the caller's prompt dst0)
+cudaError_t download_window(Lane* ln, const HostWindow& hw, uint32_t p0, uint32_t n, uint32_t dst0, cudaStream_t s) {
+    if (!n) return cudaSuccess;
+    const uint64_t L = hw.max_tokens;
+    cudaError_t e = cudaMemcpyAsync(hw.kept + dst0, ln->d_kept + p0, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && hw.cut) e = cudaMemcpyAsync(hw.cut + dst0, ln->d_cut + p0, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && hw.rows) e = cudaMemcpyAsync(hw.rows + dst0 * L, ln->d_out_ids + p0 * L, n * L * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
+    return e;
+}
 
 int fail(cfbpe_ctx*, int code, const std::string& msg) {
     tl_err = msg;
@@ -277,7 +307,7 @@ void fill_profile(Lane* ln, uint64_t n_bytes) {
         if (!ln->prof.launched[k]) continue;
         float ms = 0;
         if (cudaEventElapsedTime(&ms, ln->prof.ev[k][0], ln->prof.ev[k][1]) == cudaSuccess) p.kernel_ms[k] = ms;
-        p.kernel_launches[k] = (k == K_EMIT) ? 2 : 1;   // emit_compact + prompt_offsets
+        p.kernel_launches[k] = (k == K_EMIT) ? 2 : (k == K_WINDOW ? ln->prof.window_launches : 1);   // emit_compact + prompt_offsets
     }
     float ms = 0;
     if (cudaEventElapsedTime(&ms, ln->prof.h2d[0], ln->prof.h2d[1]) == cudaSuccess) p.h2d_ms = ms;
@@ -304,7 +334,7 @@ void fill_profile(Lane* ln, uint64_t n_bytes) {
 // buffers (dense, shard-local ranks: sub-batch k's offsets at d_out_offsets + p_k + k) and *defer gets the shard's token total.
 int run_host_pipelined(cfbpe_ctx* ctx, DeviceCtx* const* dvs, Lane* const* lns, int G, uint32_t n, const uint8_t* bytes, const uint64_t* offsets,
                        const uint8_t* vocab_ids, uint32_t* out_ids, uint64_t out_cap, uint64_t* out_offsets, uint32_t* out_counts, bool want_ids,
-                       uint64_t total, uint64_t* defer, uint32_t* cut_out, int* nc_out) {
+                       uint64_t total, uint64_t* defer, uint32_t* cut_out, int* nc_out, const HostWindow* win) {
     // ---- cut
     uint32_t cut[kMaxPipeChunks + 1];
     const int nc = plan_sub_batches(offsets, n, total, ctx->pipe_chunk, kMaxPipeChunks, cut);
@@ -344,6 +374,7 @@ int run_host_pipelined(cfbpe_ctx* ctx, DeviceCtx* const* dvs, Lane* const* lns, 
         if (len && !no_copy) CK(cudaMemcpyAsync(d_sub, bytes + o0, len, cudaMemcpyHostToDevice, hs));
         CK(cudaMemcpyAsync(ln->d_offsets + p0 + k, lns[0]->h_offs_stage + p0 + k, (static_cast<uint64_t>(nk) + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, hs));
         if (vocab_ids && nk) CK(cudaMemcpyAsync(ln->d_vocab_ids + p0, vocab_ids + p0, nk, cudaMemcpyHostToDevice, hs));
+        if (win && win->budgets && nk) CK(cudaMemcpyAsync(ln->d_budgets + p0, win->budgets + p0, nk * sizeof(uint32_t), cudaMemcpyHostToDevice, hs));
         CK(cudaEventRecord(ln->ev_h2d[k], hs));
         if (trace) CK(cudaEventRecord(ln->trace[k][0], hs));
         const int fk = k < kFrontStreams ? k : kFrontStreams - 1;
@@ -393,6 +424,7 @@ int run_host_pipelined(cfbpe_ctx* ctx, DeviceCtx* const* dvs, Lane* const* lns, 
         CK(cudaEventRecord(ln->ev_chain[k], ss));
         enqueue_emit(b, w, want_ids ? ln->d_out_ids : nullptr, ctx->max_bytes, ln->d_out_offsets + p0 + k, ln->d_out_counts + p0,
                      ss, static_cast<ProfEvents*>(nullptr));
+        if (win) enqueue_window(b, dv->vs, w, ln->d_out_offsets + p0 + k, ln->d_out_counts + p0, lane_window(ln, *win, p0), ss, static_cast<ProfEvents*>(nullptr));
         CK(cudaGetLastError());
         status_publish_kernel<<<1, 64, 0, ss>>>(ln->d_status_arr + k, ln->h_status_arr + k);
         CK(cudaEventRecord(ln->ev_done[k], ss));
@@ -419,6 +451,7 @@ int run_host_pipelined(cfbpe_ctx* ctx, DeviceCtx* const* dvs, Lane* const* lns, 
             CK(cudaMemcpyAsync(out_ids + base, ln->d_out_ids + base, st.n_tokens * sizeof(uint32_t), cudaMemcpyDeviceToHost, ds));
         if (out_offsets) CK(cudaMemcpyAsync(out_offsets + p0, ln->d_out_offsets + p0 + k, (static_cast<uint64_t>(nk) + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, ds));
         if (out_counts && nk) CK(cudaMemcpyAsync(out_counts + p0, ln->d_out_counts + p0, static_cast<uint64_t>(nk) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ds));
+        if (win) CK(download_window(ln, *win, p0, nk, p0, ds));
         if (trace) { CK(cudaEventRecord(ln->trace[k][5], ds)); host_dl[k] = host_ms(); }
     }
     for (int g = 0; g < G; ++g) {
@@ -453,30 +486,36 @@ int run_host_pipelined(cfbpe_ctx* ctx, DeviceCtx* const* dvs, Lane* const* lns, 
 // defer / cut_out / nc_out: see run_host_pipelined; the one-shot path under `defer` leaves everything on the device as ONE sub-batch.
 int run_lane(cfbpe_ctx* ctx, DeviceCtx* dv, Lane* ln, uint32_t n, const uint8_t* bytes, const uint64_t* offsets, const uint8_t* vocab_ids,
              uint32_t* out_ids, uint64_t out_cap, uint64_t* out_offsets, uint32_t* out_counts, bool want_ids, uint64_t total,
-             uint64_t* defer = nullptr, uint32_t* cut_out = nullptr, int* nc_out = nullptr) {
+             uint64_t* defer = nullptr, uint32_t* cut_out = nullptr, int* nc_out = nullptr, const HostWindow* win = nullptr) {
     CK(cudaSetDevice(dv->device));
     if (ln->ws_pending) { CK(cudaEventSynchronize(ln->ev_ws)); ln->ws_pending = false; }   // an asynchronous device-path call still owns the workspace
     const bool profiling = ctx->profiling.load();
     if (!profiling && total >= ctx->pipe_min && n >= 2)
-        return run_host_pipelined(ctx, &dv, &ln, 1, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total, defer, cut_out, nc_out);
+        return run_host_pipelined(ctx, &dv, &ln, 1, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total, defer, cut_out, nc_out, win);
     cudaStream_t s = ln->stream;
     ProfEvents* prof = profiling ? &ln->prof : nullptr;
     if (prof) { std::memset(prof->launched, 0, sizeof prof->launched); cudaEventRecord(prof->total[0], s); cudaEventRecord(prof->h2d[0], s); }
     if (total) CK(cudaMemcpyAsync(ln->d_bytes, bytes, total, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(ln->d_offsets, offsets, (static_cast<uint64_t>(n) + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
     if (vocab_ids && n) CK(cudaMemcpyAsync(ln->d_vocab_ids, vocab_ids, n, cudaMemcpyHostToDevice, s));
+    if (win && win->budgets && n) CK(cudaMemcpyAsync(ln->d_budgets, win->budgets, static_cast<uint64_t>(n) * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
     if (prof) cudaEventRecord(prof->h2d[1], s);
 
     BatchView b{ln->d_bytes, ln->d_offsets, vocab_ids ? ln->d_vocab_ids : nullptr, n, total};
     enqueue_encode(b, dv->vs, dv->uc, ln->ws, want_ids ? ln->d_out_ids : nullptr, ctx->max_bytes, ln->d_out_offsets,
                    ln->d_out_counts, static_cast<uint32_t>(dv->sm_count * 4), s, prof ? s : ln->aux_stream, prof ? s : ln->aux2_stream,
                    ln->ev_fork, ln->ev_join, ln->ev_join2, prof);
+    if (win) {
+        enqueue_window(b, dv->vs, ln->ws, ln->d_out_offsets, ln->d_out_counts, lane_window(ln, *win, 0), s, prof);
+        if (prof) prof->window_launches = (win->rows && total) ? 2 : 1;
+    }
     CK(cudaGetLastError());
     if (prof) cudaEventRecord(prof->d2h[0], s);
     CK(cudaMemcpyAsync(ln->h_status, ln->ws.status, sizeof(DeviceStatus), cudaMemcpyDeviceToHost, s));
     if (!defer) {
         if (out_offsets) CK(cudaMemcpyAsync(out_offsets, ln->d_out_offsets, (static_cast<uint64_t>(n) + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
         if (out_counts && n) CK(cudaMemcpyAsync(out_counts, ln->d_out_counts, static_cast<uint64_t>(n) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        if (win) CK(download_window(ln, *win, 0, n, 0, s));
     }
     CK(cudaStreamSynchronize(s));
     const DeviceStatus st = *ln->h_status;
@@ -510,7 +549,8 @@ __global__ void rebase_offsets_kernel(uint64_t* __restrict__ offsets, uint64_t n
 // all-gathered with NCCL (8 bytes a device: the path's only exchange), every device rebases its offsets by the totals of the
 // shards before it and downloads ids, offsets and counts straight to their final places in the caller's buffers.
 int run_multi_device(cfbpe_ctx* ctx, uint32_t n, const uint8_t* bytes, const uint64_t* offsets, const uint8_t* vocab_ids,
-                     uint32_t* out_ids, uint64_t out_cap, uint64_t* out_offsets, uint32_t* out_counts, bool want_ids, uint64_t total) {
+                     uint32_t* out_ids, uint64_t out_cap, uint64_t* out_offsets, uint32_t* out_counts, bool want_ids, uint64_t total,
+                     const HostWindow* win) {
     const uint32_t G = static_cast<uint32_t>(ctx->devs.size());
     std::vector<uint32_t> lo(G + 1, 0);
     for (uint32_t d = 1; d < G; ++d) {      // first prompt whose start is >= d * total / G
@@ -535,8 +575,10 @@ int run_multi_device(cfbpe_ctx* ctx, uint32_t n, const uint8_t* bytes, const uin
             const uint64_t o0 = offsets[p0];
             s.local_offs.resize(static_cast<size_t>(nd) + 1);
             for (uint32_t i = 0; i <= nd; ++i) s.local_offs[i] = offsets[p0 + i] - o0;
+            HostWindow sw{};                    // (a shard's budgets start at its first prompt; its results are downloaded in phase 2)
+            if (win) { sw = *win; if (sw.budgets) sw.budgets += p0; }
             s.rc = run_lane(ctx, ctx->devs[d].get(), locks[d]->ln, nd, bytes + o0, s.local_offs.data(), vocab_ids ? vocab_ids + p0 : nullptr,
-                            nullptr, 0, nullptr, nullptr, want_ids, s.local_offs[nd], &s.tokens, s.cut, &s.nc);
+                            nullptr, 0, nullptr, nullptr, want_ids, s.local_offs[nd], &s.tokens, s.cut, &s.nc, win ? &sw : nullptr);
             if (s.rc) s.err = tl_err;
         });
         for (auto& t : th) t.join();
@@ -579,6 +621,7 @@ int run_multi_device(cfbpe_ctx* ctx, uint32_t n, const uint8_t* bytes, const uin
                 if (out_offsets) ck(cudaMemcpyAsync(out_offsets + p0 + q0, src, cnt * sizeof(uint64_t), cudaMemcpyDeviceToHost, st), "offsets download");
                 if (out_counts && nk) ck(cudaMemcpyAsync(out_counts + p0 + q0, ln->d_out_counts + q0, static_cast<uint64_t>(nk) * sizeof(uint32_t), cudaMemcpyDeviceToHost, st), "counts download");
             }
+            if (win) ck(download_window(ln, *win, 0, lo[d + 1] - p0, p0, st), "window download");   // rows, kept counts, cuts: prompt-indexed, no rebase
             ck(cudaStreamSynchronize(st), "stream sync");
             uint64_t base = 0;
             for (uint32_t e = 0; e < d; ++e) base += ln->h_totals[e];
@@ -597,7 +640,7 @@ int run_multi_device(cfbpe_ctx* ctx, uint32_t n, const uint8_t* bytes, const uin
 
 // shared body of encode_batch / count_batch (host buffers)
 int run_host(cfbpe_ctx* ctx, uint32_t n, const uint8_t* bytes, const uint64_t* offsets, const uint8_t* vocab_ids,
-             uint32_t* out_ids, uint64_t out_cap, uint64_t* out_offsets, uint32_t* out_counts, bool want_ids) {
+             uint32_t* out_ids, uint64_t out_cap, uint64_t* out_offsets, uint32_t* out_counts, bool want_ids, const HostWindow* win = nullptr) {
     tl_err.clear();
     std::shared_lock<std::shared_mutex> vocabs(ctx->vocab_mu);
     uint64_t total = 0;
@@ -619,14 +662,14 @@ int run_host(cfbpe_ctx* ctx, uint32_t n, const uint8_t* bytes, const uint64_t* o
                 lns[g] = locks[g]->ln;
                 if (lns[g]->ws_pending) { CK(cudaSetDevice(dvs[g]->device)); CK(cudaEventSynchronize(lns[g]->ev_ws)); lns[g]->ws_pending = false; }
             }
-            return run_host_pipelined(ctx, dvs, lns, G, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total, nullptr, nullptr, nullptr);
+            return run_host_pipelined(ctx, dvs, lns, G, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total, nullptr, nullptr, nullptr, win);
         }
-        return run_multi_device(ctx, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total);
+        return run_multi_device(ctx, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total, win);
     }
     if (total > ctx->max_bytes) return fail(ctx, CFBPE_EINVAL, "batch exceeds max_batch_bytes of this context");
     DeviceCtx* dv = ctx->devs[0].get();
     LaneLock lk(dv);
-    return run_lane(ctx, dv, lk.ln, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total);
+    return run_lane(ctx, dv, lk.ln, n, bytes, offsets, vocab_ids, out_ids, out_cap, out_offsets, out_counts, want_ids, total, nullptr, nullptr, nullptr, win);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -637,6 +680,7 @@ void destroy_lane(Lane* ln) {
     cudaSetDevice(ln->device);
     cudaFree(ln->d_bytes); cudaFree(ln->d_offsets); cudaFree(ln->d_vocab_ids);
     cudaFree(ln->d_out_ids); cudaFree(ln->d_out_offsets); cudaFree(ln->d_out_counts);
+    cudaFree(ln->d_budgets); cudaFree(ln->d_kept); cudaFree(ln->d_cut);
     cudaFree(ln->ws.piece_bits); cudaFree(ln->ws.tok_bits); cudaFree(ln->ws.ids_by_pos);
     cudaFree(ln->ws.lscratch.rank); cudaFree(ln->ws.lscratch.aux0); cudaFree(ln->ws.lscratch.aux1);
     for (uint32_t c = 0; c < 3; ++c) cudaFree(ln->ws.miss.list[c]);
@@ -689,6 +733,9 @@ bool create_lane(Lane* ln, int device, uint64_t mb, uint64_t mp) {
     ok = ok && dmalloc(&ln->d_out_ids, mb + 1) == cudaSuccess;
     ok = ok && dmalloc(&ln->d_out_offsets, mp + 1 + kMaxPipeChunks) == cudaSuccess;
     ok = ok && dmalloc(&ln->d_out_counts, mp + 1) == cudaSuccess;
+    ok = ok && dmalloc(&ln->d_budgets, mp + 1) == cudaSuccess;
+    ok = ok && dmalloc(&ln->d_kept, mp + 1) == cudaSuccess;
+    ok = ok && dmalloc(&ln->d_cut, mp + 1) == cudaSuccess;
     ok = ok && dmalloc(&ln->ws.piece_bits, nw) == cudaSuccess;
     ok = ok && dmalloc(&ln->ws.tok_bits, nw) == cudaSuccess;
     ok = ok && dmalloc(&ln->ws.ids_by_pos, mb + 1) == cudaSuccess;
@@ -989,6 +1036,21 @@ int cfbpe_count_batch(cfbpe_ctx* ctx, uint32_t n_prompts, const uint8_t* bytes, 
     return run_host(ctx, n_prompts, bytes, offsets, vocab_ids, nullptr, 0, nullptr, out_counts, false);
 }
 
+int cfbpe_encode_truncated(cfbpe_ctx* ctx, uint32_t n_prompts, const uint8_t* bytes, const uint64_t* offsets, const uint8_t* vocab_ids,
+                           uint32_t max_tokens, uint32_t keep, uint32_t pad_id, const uint32_t* budgets, uint32_t* out_rows,
+                           uint32_t* out_kept, uint32_t* out_counts, uint64_t* out_cut) {
+    DeviceGuard restore_device;
+    if (!ctx) return CFBPE_EINVAL;
+    tl_err.clear();
+    if (!max_tokens) return fail(ctx, CFBPE_EINVAL, "max_tokens must be at least 1");
+    if (keep != CFBPE_KEEP_HEAD && keep != CFBPE_KEEP_TAIL) return fail(ctx, CFBPE_EINVAL, "keep must be CFBPE_KEEP_HEAD or CFBPE_KEEP_TAIL");
+    if (!out_kept && n_prompts) return fail(ctx, CFBPE_EINVAL, "out_kept is NULL");
+    if (out_rows && static_cast<uint64_t>(n_prompts) * max_tokens > ctx->max_bytes)
+        return fail(ctx, CFBPE_EINVAL, "n_prompts x max_tokens exceeds max_batch_bytes of this context (the rows are staged in its id buffer)");
+    const HostWindow win{max_tokens, keep, pad_id, budgets, out_rows, out_kept, out_cut};
+    return run_host(ctx, n_prompts, bytes, offsets, vocab_ids, nullptr, 0, nullptr, out_counts, false, &win);
+}
+
 int cfbpe_decode_batch(cfbpe_ctx* ctx, uint32_t n_seqs, const uint32_t* ids, const uint64_t* id_offsets,
                        const uint8_t* vocab_ids, uint8_t* out_bytes, uint64_t out_cap, uint64_t* out_offsets) {
     DeviceGuard restore_device;
@@ -1085,6 +1147,53 @@ int cfbpe_encode_batch_device(cfbpe_ctx* ctx, uint32_t n_prompts, const uint8_t*
         if (st.bad_vocab) return fail(ctx, CFBPE_ENOENT, "a prompt names a vocabulary that is not loaded");
         if (st.bad_utf8) return fail(ctx, CFBPE_EILSEQ, "a prompt holds malformed UTF-8");
         if (d_out_ids && st.n_tokens > out_cap) return fail(ctx, CFBPE_ENOSPC, "out_cap too small: need " + std::to_string(st.n_tokens) + " ids");
+    }
+    return CFBPE_OK;
+}
+
+int cfbpe_encode_truncated_device(cfbpe_ctx* ctx, uint32_t n_prompts, const uint8_t* d_bytes, uint64_t total_bytes,
+                                  const uint64_t* d_offsets, const uint8_t* d_vocab_ids, uint32_t max_tokens, uint32_t keep, uint32_t pad_id,
+                                  const uint32_t* d_budgets, uint32_t* d_out_rows, uint32_t* d_out_kept, uint32_t* d_out_counts,
+                                  uint64_t* d_out_cut, void* stream) {
+    DeviceGuard restore_device;
+    if (!ctx) return CFBPE_EINVAL;
+    tl_err.clear();
+    std::shared_lock<std::shared_mutex> vocabs(ctx->vocab_mu);
+    if (n_prompts > ctx->max_prompts || total_bytes > ctx->max_bytes) return fail(ctx, CFBPE_EINVAL, "batch exceeds the limits of this context");
+    if (!d_offsets || !d_out_kept || (total_bytes && !d_bytes)) return fail(ctx, CFBPE_EINVAL, "device pointer is NULL");
+    if (!max_tokens) return fail(ctx, CFBPE_EINVAL, "max_tokens must be at least 1");
+    if (keep != CFBPE_KEEP_HEAD && keep != CFBPE_KEEP_TAIL) return fail(ctx, CFBPE_EINVAL, "keep must be CFBPE_KEEP_HEAD or CFBPE_KEEP_TAIL");
+    if (!ctx->vocabs[0].loaded && !d_vocab_ids) return fail(ctx, CFBPE_ENOENT, "vocab 0 is not loaded");
+    if (!ctx->loaded_mask) return fail(ctx, CFBPE_ENOENT, "no vocabulary is loaded");
+    DeviceCtx* dv = ctx->devs[0].get();
+    { int cur = -1; if (cudaGetDevice(&cur) == cudaSuccess) for (auto& d : ctx->devs) if (d->device == cur) dv = d.get(); }
+    LaneLock lk(dv);
+    Lane* ln = lk.ln;
+    CK(cudaSetDevice(dv->device));
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (ln->ws_pending) CK(cudaStreamWaitEvent(s, ln->ev_ws, 0));
+    const bool profiling = ctx->profiling.load();
+    ProfEvents* prof = profiling ? &ln->prof : nullptr;
+    if (prof) { std::memset(prof->launched, 0, sizeof prof->launched); cudaEventRecord(prof->total[0], s); cudaEventRecord(prof->h2d[0], s); cudaEventRecord(prof->h2d[1], s); }
+    // the token offsets and counts the window reads go to the lane's own buffers; the caller's counts are a copy of them
+    BatchView b{d_bytes, d_offsets, d_vocab_ids, n_prompts, total_bytes};
+    enqueue_encode(b, dv->vs, dv->uc, ln->ws, nullptr, 0, ln->d_out_offsets, ln->d_out_counts,
+                   static_cast<uint32_t>(dv->sm_count * 4), s, prof ? s : ln->aux_stream, prof ? s : ln->aux2_stream,
+                   ln->ev_fork, ln->ev_join, ln->ev_join2, prof);
+    const WindowView win{max_tokens, keep, pad_id, d_budgets, d_out_rows, d_out_kept, d_out_counts, d_out_cut};
+    enqueue_window(b, dv->vs, ln->ws, ln->d_out_offsets, ln->d_out_counts, win, s, prof);
+    if (prof) prof->window_launches = (d_out_rows && total_bytes) ? 2 : 1;
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(ln->ev_ws, s));
+    ln->ws_pending = true;
+    ln->dev_out_cap = 0;
+    ln->dev_want_ids = false;
+    tl_device_lane = ln;
+    if (prof) {
+        cudaEventRecord(prof->d2h[0], s); cudaEventRecord(prof->d2h[1], s); cudaEventRecord(prof->total[1], s);
+        CK(cudaMemcpyAsync(ln->h_status, ln->ws.status, sizeof(DeviceStatus), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        fill_profile(ln, total_bytes);
     }
     return CFBPE_OK;
 }

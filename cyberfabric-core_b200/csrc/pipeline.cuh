@@ -9,6 +9,7 @@
 //   CFBPE_FORK(main, aux, ev) / CFBPE_JOIN(main, aux, ev)   make aux wait for main / main wait for aux
 #pragma once
 #include "bpe_kernels.cuh"
+#include "window.cuh"
 
 namespace cfbpe {
 
@@ -56,7 +57,7 @@ constexpr uint32_t kLongCtasPerSm = CFBPE_LONG_CTAS;
 #endif
 constexpr uint32_t kListCtasPerSm = CFBPE_LIST_CTAS;   // K2c CTAs (64 KB of shared memory each) per SM
 
-enum KernelIdx { K_SPLIT = 0, K_ENCODE = 1, K_LONG = 2, K_COUNT = 3, K_SCAN = 4, K_EMIT = 5, K_LIST = 6, K_LONGSCAN = 7, K_MERGE = 8 };
+enum KernelIdx { K_SPLIT = 0, K_ENCODE = 1, K_LONG = 2, K_COUNT = 3, K_SCAN = 4, K_EMIT = 5, K_LIST = 6, K_LONGSCAN = 7, K_MERGE = 8, K_WINDOW = 9 };
 
 inline uint64_t n_flag_words(uint64_t total_bytes) { return (total_bytes + 31) >> 5; }
 inline uint32_t n_scan_tiles(uint64_t total_bytes) {
@@ -176,6 +177,22 @@ inline void enqueue_back(const BatchView& b, const Workspace& w, uint32_t* out_i
     enqueue_count(b, w, stream, prof);
     enqueue_scan(b, w, stream, prof, token_base);
     enqueue_emit(b, w, out_ids, out_cap, out_offsets, out_counts, stream, prof);
+}
+
+// window (truncated encode, after enqueue_emit has written the token offsets and counts of the (sub-)batch): tok_off[p] = rank of
+// prompt p's first token, counts[p] = its token count (prompt_offsets_kernel's outputs).  Rows are emitted only when win.rows is set.
+template <typename Stream, typename Prof>
+inline void enqueue_window(const BatchView& b, const VocabSet& vs, const Workspace& w, const uint64_t* tok_off, const uint32_t* counts,
+                           const WindowView& win, Stream stream, Prof* prof) {
+    if (!b.n_prompts) return;
+    CFBPE_MARK(prof, K_WINDOW, stream, true);
+    CFBPE_LAUNCH(window_select_kernel, static_cast<unsigned>((static_cast<uint64_t>(b.n_prompts) + 7) / 8), 256, stream,    // a warp per prompt
+                 b, vs, w.tok_bits, w.piece_bits, w.ids_by_pos, counts, win);
+    if (b.total_bytes && win.rows) {
+        CFBPE_LAUNCH(emit_window_kernel, n_scan_tiles(b.total_bytes), 256, stream, w.tok_bits, w.piece_bits, n_flag_words(b.total_bytes),
+                     w.tile_base, w.dense, w.ids_by_pos, b, w.block_prompt, tok_off, counts, win);
+    }
+    CFBPE_MARK(prof, K_WINDOW, stream, false);
 }
 
 // The whole path.  `aux` / `aux2` are streams of their own for the two long-piece kernels (pass the main stream to run everything

@@ -25,6 +25,8 @@
  *                                  and check_budget / report_usage (modules/llm-gateway/docs/DESIGN.md:833-855).
  *   cfbpe_encode_batch_device      same path with inputs/outputs already resident in HBM
  *                                  (for callers that keep token ids on the GPU).
+ *   cfbpe_encode_truncated[_device] a prompt cut to a token budget: the request may not exceed the provider's context window
+ *                                  (modules/llm-gateway/docs/DESIGN.md:102-106); fixed-length id rows and the byte cut of each prompt.
  *
  * Conventions (SURVEY.md section 8(b)): 0 = ok, negative errno-style code = error; the caller
  * owns every buffer it passes and the library never retains a caller pointer past return;
@@ -88,7 +90,8 @@ typedef struct cfbpe_config {
                                  ABI version 1 (24 bytes) still works, and gets one device and one workspace */
     int32_t device;           /* CUDA device ordinal (used when n_devices == 0) */
     uint64_t max_batch_bytes; /* largest packed prompt buffer one DEVICE takes in one call (0 = 256 MiB) */
-    uint32_t max_prompts;     /* largest n_prompts of one call (0 = 1 Mi) */
+    uint32_t max_prompts;     /* largest n_prompts of one call (0 = 1 Mi); each workspace holds 16 bytes of device memory per prompt
+                                 for the budgets, kept counts and cuts of cfbpe_encode_truncated */
     uint32_t flags;           /* reserved, 0 */
     /* SURVEY.md section 8(b): cfbpe_create(cfg: devices[], n_devices, ...) */
     int32_t devices[CFBPE_MAX_DEVICES]; /* CUDA ordinals of a multi-device context */
@@ -112,7 +115,8 @@ typedef struct cfbpe_vocab_info {
 /* per-call device timings, filled when profiling is on (cfbpe_profile_enable) */
 #define CFBPE_NUM_KERNELS 10
 typedef struct cfbpe_profile {
-    float kernel_ms[CFBPE_NUM_KERNELS]; /* 0 pretok_split, 1 bpe_encode, 2 bpe_long, 3 flag_count, 4 tile_scan, 5 emit_compact (+ offsets), 6 bpe_list, 7 long_scan, 8 bpe_merge, 9 reserved */
+    float kernel_ms[CFBPE_NUM_KERNELS]; /* 0 pretok_split, 1 bpe_encode, 2 bpe_long, 3 flag_count, 4 tile_scan, 5 emit_compact (+ offsets), 6 bpe_list, 7 long_scan, 8 bpe_merge,
+                                           9 window (cfbpe_encode_truncated only: window_select + emit_window; 0 otherwise) */
     uint32_t kernel_launches[CFBPE_NUM_KERNELS];
     float h2d_ms, d2h_ms, total_ms;
     uint64_t n_tokens, n_bytes, n_long_pieces;
@@ -153,6 +157,29 @@ CFBPE_API int cfbpe_encode_batch(cfbpe_ctx *ctx, uint32_t n_prompts, const uint8
 CFBPE_API int cfbpe_count_batch(cfbpe_ctx *ctx, uint32_t n_prompts, const uint8_t *bytes, const uint64_t *offsets,
                       const uint8_t *vocab_ids, uint32_t *out_counts);
 
+/* Truncated encode: every prompt cut to a token budget, as fixed-length rows of ids.
+ * Prompt i has c_i tokens (its full encode_ordinary) and keeps k_i = min(c_i, budgets[i], max_tokens) of them (budgets may be
+ * NULL: max_tokens for every prompt; max_tokens >= 1).
+ *   keep = CFBPE_KEEP_HEAD: ids[0 : k_i]; out_cut[i] = the byte offset inside the prompt where token k_i starts, or the prompt's
+ *          length when nothing was dropped; the kept tokens cover exactly prompt[0 : cut].
+ *   keep = CFBPE_KEEP_TAIL: ids[c_i - k_i : c_i]; out_cut[i] = where the first kept token starts, or 0 when nothing was dropped;
+ *          the kept tokens cover exactly prompt[cut : len].
+ * out_rows (may be NULL: no id leaves the device) is n_prompts x max_tokens uint32, row-major: row i holds the k_i kept ids
+ * left-aligned, then pad_id up to max_tokens.  out_kept[i] = k_i (required), out_counts[i] = c_i (may be NULL), out_cut[i]
+ * (may be NULL).
+ * The kept ids are a slice of the full encoding.  Re-encoding the kept bytes need not give the same ids: the pre-tokenizer's
+ * lookahead (\s+(?!\S)) sees different text at the cut.  And a cut may fall inside a multi-byte UTF-8 character (byte-level tokens
+ * split CJK characters and emoji): out_cut is the token boundary exactly as it is, never moved to a character boundary.
+ * Errors as cfbpe_encode_batch (EILSEQ, ENOENT, EINVAL for bad offsets and limits), and CFBPE_EINVAL for max_tokens == 0, an
+ * unknown keep, a NULL out_kept, or, with out_rows, n_prompts x max_tokens > max_batch_bytes (the rows are staged in the
+ * context's id buffer).  Never CFBPE_ENOSPC: the caller sizes the rows. */
+#define CFBPE_KEEP_HEAD 0u
+#define CFBPE_KEEP_TAIL 1u
+CFBPE_API int cfbpe_encode_truncated(cfbpe_ctx *ctx, uint32_t n_prompts, const uint8_t *bytes, const uint64_t *offsets,
+                                     const uint8_t *vocab_ids, uint32_t max_tokens, uint32_t keep, uint32_t pad_id,
+                                     const uint32_t *budgets, uint32_t *out_rows, uint32_t *out_kept, uint32_t *out_counts,
+                                     uint64_t *out_cut);
+
 /* Decode (SURVEY.md section 8(f) item 2; tiktoken CoreBPE.decode_bytes): out_bytes = the concatenation of the tokens' bytes.
  * ids: the packed token ids of n_seqs sequences, id_offsets[n_seqs + 1] their boundaries (in ids), vocab_ids[n_seqs] or NULL.
  * out_offsets[n_seqs + 1]: byte boundaries of the decoded sequences in out_bytes.  CFBPE_ENOSPC if out_cap is too small
@@ -172,6 +199,14 @@ CFBPE_API int cfbpe_encode_batch_device(cfbpe_ctx *ctx, uint32_t n_prompts, cons
                               const uint64_t *d_offsets, const uint8_t *d_vocab_ids, uint32_t *d_out_ids,
                               uint64_t out_cap, uint64_t *d_out_offsets, uint32_t *d_out_counts,
                               uint64_t *n_tokens, void *stream);
+/* cfbpe_encode_truncated on device-resident buffers, asynchronous as cfbpe_encode_batch_device (d_bytes padded by 32 readable
+ * bytes; errors through cfbpe_device_status).  d_budgets, d_out_rows, d_out_counts, d_out_cut may be NULL; no limit on
+ * n_prompts x max_tokens (the rows are the caller's buffer).  The context's own offset and count buffers hold the token offsets
+ * the window reads. */
+CFBPE_API int cfbpe_encode_truncated_device(cfbpe_ctx *ctx, uint32_t n_prompts, const uint8_t *d_bytes, uint64_t total_bytes,
+                                            const uint64_t *d_offsets, const uint8_t *d_vocab_ids, uint32_t max_tokens,
+                                            uint32_t keep, uint32_t pad_id, const uint32_t *d_budgets, uint32_t *d_out_rows,
+                                            uint32_t *d_out_kept, uint32_t *d_out_counts, uint64_t *d_out_cut, void *stream);
 /* Synchronise `stream` and return the status word of the last device call (0, CFBPE_EILSEQ, CFBPE_ENOSPC). */
 CFBPE_API int cfbpe_device_status(cfbpe_ctx *ctx, void *stream);
 

@@ -21,6 +21,8 @@ pub const CFBPE_EILSEQ: c_int = -84;
 pub const CFBPE_FORMAT_TIKTOKEN: u32 = 0;
 pub const CFBPE_FORMAT_TEKKEN_JSON: u32 = 1;
 pub const CFBPE_MAX_VOCABS: u32 = 8;
+pub const CFBPE_KEEP_HEAD: u32 = 0;
+pub const CFBPE_KEEP_TAIL: u32 = 1;
 pub const CFBPE_MAX_DEVICES: usize = 8;
 
 #[repr(C)]
@@ -76,6 +78,13 @@ extern "C" {
                                      d_offsets: *const u64, d_vocab_ids: *const u8, d_out_ids: *mut u32, out_cap: u64,
                                      d_out_offsets: *mut u64, d_out_counts: *mut u32, n_tokens: *mut u64,
                                      stream: *mut c_void) -> c_int;
+    pub fn cfbpe_encode_truncated(ctx: *mut cfbpe_ctx, n_prompts: u32, bytes: *const u8, offsets: *const u64, vocab_ids: *const u8,
+                                  max_tokens: u32, keep: u32, pad_id: u32, budgets: *const u32, out_rows: *mut u32,
+                                  out_kept: *mut u32, out_counts: *mut u32, out_cut: *mut u64) -> c_int;
+    pub fn cfbpe_encode_truncated_device(ctx: *mut cfbpe_ctx, n_prompts: u32, d_bytes: *const u8, total_bytes: u64,
+                                         d_offsets: *const u64, d_vocab_ids: *const u8, max_tokens: u32, keep: u32, pad_id: u32,
+                                         d_budgets: *const u32, d_out_rows: *mut u32, d_out_kept: *mut u32, d_out_counts: *mut u32,
+                                         d_out_cut: *mut u64, stream: *mut c_void) -> c_int;
     pub fn cfbpe_device_status(ctx: *mut cfbpe_ctx, stream: *mut c_void) -> c_int;
     pub fn cfbpe_host_alloc(ctx: *mut cfbpe_ctx, size: usize) -> *mut c_void;
     pub fn cfbpe_host_free(ctx: *mut cfbpe_ctx, ptr: *mut c_void);
@@ -95,6 +104,16 @@ pub struct Encoded {
     pub ids: Vec<u32>,
     pub offsets: Vec<u64>,
     pub counts: Vec<u32>,
+}
+
+/// Result of [`Ctx::encode_truncated`]: `n x max_tokens` rows (kept ids left-aligned, then `pad_id`; empty without ids),
+/// the kept and untruncated counts, and the byte offset of the cut inside each prompt.
+#[derive(Debug, Default)]
+pub struct Truncated {
+    pub rows: Vec<u32>,
+    pub kept: Vec<u32>,
+    pub counts: Vec<u32>,
+    pub cut: Vec<u64>,
 }
 
 /// Safe owner of one `cfbpe_ctx`.  The context is internally synchronised (header: "safe to call concurrently from several
@@ -200,6 +219,37 @@ impl Ctx {
         self.check(rc)?;
         counts.truncate(n as usize);
         Ok(counts)
+    }
+
+    /// Every prompt cut to `min(count, budgets[i], max_tokens)` tokens, its first ones (`CFBPE_KEEP_HEAD`) or its last ones
+    /// (`CFBPE_KEEP_TAIL`); `want_ids == false`: kept counts and cuts only, no id leaves the device.
+    #[allow(clippy::too_many_arguments)]
+    pub fn encode_truncated(&self, bytes: &[u8], offsets: &[u64], vocab_ids: Option<&[u8]>, max_tokens: u32, keep: u32, pad_id: u32,
+                            budgets: Option<&[u32]>, want_ids: bool) -> Result<Truncated, NativeError> {
+        let n = Self::check_inputs(bytes.len(), offsets, vocab_ids)?;
+        if budgets.is_some_and(|b| b.len() != n as usize) {
+            return Err(NativeError { code: CFBPE_EINVAL, message: "budgets needs one entry per prompt".to_owned() });
+        }
+        let m = (n as usize).max(1);
+        let mut out = Truncated {
+            rows: if want_ids { vec![0; n as usize * max_tokens as usize] } else { Vec::new() },
+            kept: vec![0; m],
+            counts: vec![0; m],
+            cut: vec![0; m],
+        };
+        // SAFETY: all buffers are valid for the sizes passed (rows: n x max_tokens); the library checks max_tokens, keep and the
+        // row budget of the context before it writes anything.
+        let rc = unsafe {
+            cfbpe_encode_truncated(self.0.as_ptr(), n, bytes.as_ptr(), offsets.as_ptr(), vocab_ids.map_or(std::ptr::null(), <[u8]>::as_ptr),
+                                   max_tokens, keep, pad_id, budgets.map_or(std::ptr::null(), <[u32]>::as_ptr),
+                                   if want_ids { out.rows.as_mut_ptr() } else { std::ptr::null_mut() }, out.kept.as_mut_ptr(),
+                                   out.counts.as_mut_ptr(), out.cut.as_mut_ptr())
+        };
+        self.check(rc)?;
+        out.kept.truncate(n as usize);
+        out.counts.truncate(n as usize);
+        out.cut.truncate(n as usize);
+        Ok(out)
     }
 
     /// ids -> bytes (tiktoken `decode_bytes`); grows the output once when the library reports `CFBPE_ENOSPC`.

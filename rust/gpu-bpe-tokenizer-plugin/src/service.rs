@@ -4,10 +4,10 @@ use std::collections::HashMap;
 use std::sync::Arc;
 
 use async_trait::async_trait;
-use cfbpe_sys::{Ctx, NativeError};
+use cfbpe_sys::{Ctx, NativeError, CFBPE_KEEP_HEAD, CFBPE_KEEP_TAIL};
 use llm_gateway_sdk::{
-    CountTokensRequest, DecodeBatchRequest, DecodeBatchResponse, EncodeBatchRequest, EncodeBatchResponse, TokenizerError,
-    TokenizerPluginClient, VocabRef,
+    CountTokensRequest, DecodeBatchRequest, DecodeBatchResponse, EncodeBatchRequest, EncodeBatchResponse, Keep, TokenizerError,
+    TokenizerPluginClient, TruncateBatchRequest, TruncateBatchResponse, VocabRef,
 };
 use modkit_security::SecurityContext;
 use sha2::{Digest, Sha256};
@@ -136,6 +136,20 @@ impl TokenizerPluginClient for Service {
             .map_err(|e| TokenizerError::Internal(e.to_string()))?
             .map_err(map_native)?;
         Ok(DecodeBatchResponse { bytes, offsets })
+    }
+
+    async fn truncate_batch(&self, _ctx: &SecurityContext, req: TruncateBatchRequest) -> Result<TruncateBatchResponse, TokenizerError> {
+        let n = req.offsets.len().saturating_sub(1);
+        let vid = self.vocab_ids(&req.vocab, req.vocabs_per_prompt.as_deref(), req.vocab_index.as_deref(), n)?;
+        let keep = match req.keep { Keep::Head => CFBPE_KEEP_HEAD, Keep::Tail => CFBPE_KEEP_TAIL };
+        let native = self.native.clone();
+        let out = tokio::task::spawn_blocking(move || {
+            native.encode_truncated(&req.bytes, &req.offsets, vid.as_deref(), req.max_tokens, keep, req.pad_id, req.budgets.as_deref(), req.want_ids)
+        })
+        .await
+        .map_err(|e| TokenizerError::Internal(e.to_string()))?
+        .map_err(map_native)?;
+        Ok(TruncateBatchResponse { rows: out.rows, kept: out.kept, counts: out.counts, cut: out.cut })
     }
 }
 

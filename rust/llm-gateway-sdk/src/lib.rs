@@ -19,6 +19,6 @@ pub use api::TokenizerClient;
 pub use error::TokenizerError;
 pub use gts::TokenizerPluginSpecV1;
 pub use models::{
-    ChatTemplate, CountTokensRequest, DecodeBatchRequest, DecodeBatchResponse, EncodeBatchRequest, EncodeBatchResponse, SpecialTokens, Usage, VocabRef,
+    ChatTemplate, CountTokensRequest, DecodeBatchRequest, DecodeBatchResponse, EncodeBatchRequest, EncodeBatchResponse, Keep, SpecialTokens, TruncateBatchRequest, TruncateBatchResponse, Usage, VocabRef,
 };
 pub use plugin_api::TokenizerPluginClient;

@@ -45,6 +45,46 @@ pub struct CountTokensRequest {
     pub vocab_index: Option<Vec<u8>>,
 }
 
+/// Which end of a prompt a truncation keeps.
+#[derive(Debug, Clone, Copy, PartialEq, Eq, Default, Serialize, Deserialize)]
+#[serde(rename_all = "snake_case")]
+pub enum Keep {
+    #[default]
+    Head,
+    Tail,
+}
+
+/// Every prompt cut to `k_i = min(count_i, budgets[i], max_tokens)` tokens: the first `k_i` (`Keep::Head`) or the last (`Keep::Tail`)
+/// of its full encoding.  The kept ids are a slice of that encoding (re-encoding the kept bytes need not give the same ids), and the
+/// cut is the token boundary as it is, possibly inside a multi-byte UTF-8 character.
+#[derive(Debug, Clone)]
+pub struct TruncateBatchRequest {
+    pub vocab: VocabRef,
+    pub bytes: Bytes,
+    pub offsets: Vec<u64>,
+    /// ids per row, >= 1
+    pub max_tokens: u32,
+    pub keep: Keep,
+    pub pad_id: u32,
+    /// one budget per prompt, or `max_tokens` for every prompt
+    pub budgets: Option<Vec<u32>>,
+    /// false: kept counts and cuts only, no id leaves the device
+    pub want_ids: bool,
+    pub vocabs_per_prompt: Option<Vec<VocabRef>>,
+    pub vocab_index: Option<Vec<u8>>,
+}
+
+#[derive(Debug, Clone, Default)]
+pub struct TruncateBatchResponse {
+    /// `n x max_tokens`, row-major: prompt i's kept ids left-aligned, then `pad_id` (empty when `want_ids` is false)
+    pub rows: Vec<u32>,
+    pub kept: Vec<u32>,
+    /// the untruncated counts
+    pub counts: Vec<u32>,
+    /// byte offset of the cut inside prompt i: `Head` keeps `prompt[..cut]`, `Tail` keeps `prompt[cut..]`
+    pub cut: Vec<u64>,
+}
+
 #[derive(Debug, Clone)]
 pub struct DecodeBatchRequest {
     pub vocab: VocabRef,

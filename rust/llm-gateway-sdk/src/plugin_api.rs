@@ -4,7 +4,10 @@ use async_trait::async_trait;
 use modkit_security::SecurityContext;
 
 use crate::error::TokenizerError;
-use crate::models::{CountTokensRequest, DecodeBatchRequest, DecodeBatchResponse, EncodeBatchRequest, EncodeBatchResponse};
+use crate::models::{
+    CountTokensRequest, DecodeBatchRequest, DecodeBatchResponse, EncodeBatchRequest, EncodeBatchResponse, TruncateBatchRequest,
+    TruncateBatchResponse,
+};
 
 /// Each plugin registers this trait with a scoped `ClientHub` entry using its GTS instance id as the scope.  Clients are
 /// `Arc<dyn … + Send + Sync>` shared by all tokio tasks (`libs/modkit/src/client_hub.rs:142-165`): calls are concurrent and
@@ -22,4 +25,8 @@ pub trait TokenizerPluginClient: Send + Sync {
 
     /// ids -> bytes; `InvalidInput` for an id outside its vocabulary.
     async fn decode_batch(&self, ctx: &SecurityContext, req: DecodeBatchRequest) -> Result<DecodeBatchResponse, TokenizerError>;
+
+    /// Every prompt cut to a token budget: fixed-length id rows, kept and full counts, the byte cut of each prompt; the errors
+    /// of `encode_batch`, and `InvalidInput` for `max_tokens == 0` or rows beyond the plugin's batch limit.
+    async fn truncate_batch(&self, ctx: &SecurityContext, req: TruncateBatchRequest) -> Result<TruncateBatchResponse, TokenizerError>;
 }
